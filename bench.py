@@ -28,6 +28,31 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 N_SERIES, SERIES_LEN, PREFIX_IDS, PROMPT_IDS = 8, 256, 46, 64
+PROMPT_POSITIONS = N_SERIES * (PREFIX_IDS + 2 + SERIES_LEN // 16) + PROMPT_IDS          # 576 merged positions per prompt
+DUMP_BYTES = 64 << 20                                                                   # --dump-outputs: at most this much in all
+
+
+def seq_capacity(max_new, prompt_positions=PROMPT_POSITIONS):
+    """KV positions per sequence of a benchmark model: 1024, or more when --steps asks for more new tokens than that holds."""
+    return max(1024, -(-(prompt_positions + max_new) // 64) * 64)
+
+
+def dump_outputs(out_dir, logits, tokens):
+    """--dump-outputs: what the timed decode path hands its caller after its last step -- the next-token logits of every sequence
+    [B, V] and every greedy token generated so far [B, n] -- as out_dir/logits.npy (float32) and out_dir/tokens.npy (float64, exact).
+    Logits larger than what DUMP_BYTES leaves keep a fixed, seeded sample of vocabulary columns (the same columns for every
+    sequence), whose indices go to out_dir/logits_columns.npy.  Returns the names written."""
+    os.makedirs(out_dir, exist_ok=True)
+    tok = tokens.cpu().numpy().astype(np.float64)
+    lg = logits.float().cpu().numpy()
+    out = {"tokens": tok, "logits": lg}
+    room = (DUMP_BYTES - tok.nbytes) // (4 * lg.shape[0] + 8)
+    if lg.shape[1] > room:
+        cols = np.sort(np.random.default_rng(0).choice(lg.shape[1], room, replace=False))
+        out["logits"], out["logits_columns"] = np.ascontiguousarray(lg[:, cols]), cols.astype(np.float64)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return sorted(out)
 
 
 def peaks():
@@ -538,10 +563,10 @@ def measure_w4(cfg, steps, warmup, hbm_peak, batches=(1, 8, 32)):
     encoder stay bf16) decodes the benchmark prompts through the packed weights (cts_gemm_w4_mma) and through its own dequantised bf16
     copy: ms per step of both from CUDA events over graph replays, greedy agreement between the two."""
     from chatts_b200.model import ChatTSForCausalLM
-    model = ChatTSForCausalLM.from_synthetic(cfg, seed=1234, max_batch=max(batches), max_seq_len=1024, page_size=64)
+    max_new = steps + warmup + 8
+    model = ChatTSForCausalLM.from_synthetic(cfg, seed=1234, max_batch=max(batches), max_seq_len=seq_capacity(max_new), page_size=64)
     model.quantize_w4_synthetic(group_size=128)
     w4 = model.w4
-    max_new = steps + warmup + 8
 
     def run(batch):
         enc = make_batch(cfg, batch)
@@ -616,7 +641,7 @@ def run_b200(args):
     hbm_peak, peak_src = peaks()
     max_new = args.steps + args.warmup + 8
     model = ChatTSForCausalLM.from_synthetic(cfg, seed=1234, tp_rank=rank, tp_size=world, max_batch=max(args.batch, 1),
-                                             max_seq_len=1024, page_size=64, use_cuda_graph=not args.no_graph)
+                                             max_seq_len=seq_capacity(max_new), page_size=64, use_cuda_graph=not args.no_graph)
     ctx = model.ctx
 
     def sync_all():
@@ -662,11 +687,15 @@ def run_b200(args):
             ctx_end = int(lay.lens.max()) + n_tok
             import hashlib
             tok_sha = hashlib.sha1(st.out_tokens[:, :n_tok].to(torch.int32).cpu().numpy().tobytes()).hexdigest()[:16]
+            if args.dump_outputs and batch == args.batch:
+                logits = model._gather_vocab(st.logits[:batch])         # every rank takes part in the gather of the vocab shards
+                if rank == 0:
+                    dumped.extend(dump_outputs(args.dump_outputs, logits, st.out_tokens[:batch, :n_tok]))
         finally:
             model.pool.release(held)
         return ms, per_step_launches, ctx_end, tok_sha
 
-    results = {}
+    results, dumped = {}, []
     with ClockSampler(local) as clk:
         batches = [args.batch] if args.only_batch else sorted(set(b for b in (1, 8, args.batch) if b <= args.batch))
         for b in batches:
@@ -851,6 +880,8 @@ def run_b200(args):
         line["tokens_sha1"] = main.get("tokens_sha1")          # hash of every greedy token the measured batch produced (probe: equality across variants)
         if probe_record is not None:
             line["config"]["decode_variant_probe"] = probe_record
+        if args.dump_outputs:
+            line["dumped_outputs"] = {"dir": args.dump_outputs, "names": dumped, "batch": args.batch}
         if world > 1:
             line["tp_parity"] = tp_gate
             # per rank and step: 2 row-parallel tails per layer, each a two-shot exchange with the flags inside the data (LL):
@@ -880,6 +911,9 @@ def main():
     ap.add_argument("--no-w4", action="store_true", help="skip the GPTQ-Int4 side block (third model instance with 4-bit projections)")
     ap.add_argument("--no-config4", action="store_true", help="skip the BASELINE configs[3] side block (second model instance, 30 x 512-point prompts)")
     ap.add_argument("--no-probe", action="store_true", help="(default) the default decode path is measured as is")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the measured batch's last-step logits and its greedy tokens as DIR/<name>.npy (float32 / "
+                         "float64, at most 64 MB; seeded inputs, so two builds can be compared output for output)")
     ap.add_argument("--probe", action="store_true", help="guarded child-process probe of the cluster-fused decode variants (round 1; measured slower at b = 32 on a B200, "
                                                         "profiles/r2_decode_variants_ab.txt, so no longer on by default)")
     args = ap.parse_args()

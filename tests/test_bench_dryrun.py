@@ -6,6 +6,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -13,8 +14,9 @@ CONTRACT = ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step
             "config", "clocks", "e2e", "gpu_launches", "roofline")
 
 
-def _run(which):
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "tools", "dryrun_bench.py"), which], capture_output=True, text=True, timeout=600, cwd=ROOT)
+def _run(which, *flags):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "tools", "dryrun_bench.py"), which, *flags], capture_output=True, text=True, timeout=600,
+                       cwd=ROOT)
     assert r.returncode == 0, r.stderr[-3000:]
     lines = [ln for ln in r.stdout.strip().split("\n") if ln.startswith("{")]
     assert len(lines) == 1, r.stdout[-2000:]
@@ -108,3 +110,47 @@ def test_probe_child_run_parses_the_json_line_and_survives_failures(tmp_path, mo
     assert "error" in bench._probe_run(1, args) and "rc=134" in bench._probe_run(1, args)["error"]
     monkeypatch.setattr(bench, "__file__", str(slow))
     assert "error" in bench._probe_run(1, args, timeout=1)
+
+
+def test_dump_outputs_writes_the_last_timed_step(tmp_path):
+    """--dump-outputs: the measured batch's last-step logits (float32) and its greedy tokens (float64) land in DIR; --steps sets how many
+    timed steps ran (three more steps = three more tokens), and the inputs are the same from run to run (the shorter run's tokens are a
+    prefix of the longer run's)."""
+    runs = {}
+    for steps in (2, 5):
+        out = tmp_path / f"steps{steps}"
+        d = _run("decode", "--dump-outputs", str(out), "--steps", str(steps), "--no-w4", "--no-config4")
+        assert d["steps"] == steps and d["dumped_outputs"]["names"] == ["logits", "tokens"]
+        lg, tok = np.load(out / "logits.npy"), np.load(out / "tokens.npy")
+        assert lg.dtype == np.float32 and tok.dtype == np.float64 and np.isfinite(lg).all()
+        assert lg.shape[0] == tok.shape[0] == d["config"]["batch"] and lg.shape[1] == 152064
+        assert sum(f.stat().st_size for f in out.iterdir()) <= 64 << 20
+        runs[steps] = tok
+    assert runs[5].shape[1] - runs[2].shape[1] == 3
+    assert np.array_equal(runs[5][:, : runs[2].shape[1]], runs[2])
+
+
+def test_dump_outputs_keeps_a_fixed_sample_of_columns_within_the_budget(tmp_path, monkeypatch):
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    lg, tok = torch.randn(3, 5000, dtype=torch.bfloat16), torch.randint(0, 5000, (3, 7), dtype=torch.int32)
+    monkeypatch.setattr(bench, "DUMP_BYTES", 20000)
+    for sub in ("a", "b"):
+        assert bench.dump_outputs(str(tmp_path / sub), lg, tok) == ["logits", "logits_columns", "tokens"]
+    got = {n: np.load(tmp_path / "a" / f"{n}.npy") for n in ("logits", "logits_columns", "tokens")}
+    assert sum(a.nbytes for a in got.values()) <= 20000
+    cols = got["logits_columns"].astype(np.int64)
+    assert np.all(np.diff(cols) > 0) and got["logits"].shape == (3, cols.size)
+    assert np.array_equal(got["logits"], lg.float().numpy()[:, cols]) and np.array_equal(got["tokens"], tok.numpy())
+    for n, a in got.items():
+        assert np.array_equal(np.load(tmp_path / "b" / f"{n}.npy"), a), n
+
+
+def test_the_kv_cache_makes_room_for_every_requested_step():
+    sys.path.insert(0, ROOT)
+    import bench
+    assert bench.seq_capacity(20 + 5 + 8) == 1024                      # the size every recorded run used
+    for steps in (430, 500, 2000):
+        cap = bench.seq_capacity(steps + 3 + 8)
+        assert cap % 64 == 0 and cap >= bench.PROMPT_POSITIONS + steps + 3 + 8

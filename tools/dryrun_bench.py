@@ -1,8 +1,8 @@
 #!/usr/bin/env python
 """Dry run of the benchmark drivers on a machine WITHOUT a GPU (TEST INFRASTRUCTURE ONLY -- not a measurement).
 
-    python tools/dryrun_bench.py decode      # bench.py's B200 arm
-    python tools/dryrun_bench.py lora        # tools/bench_lora.py
+    python tools/dryrun_bench.py decode [bench.py flags]      # bench.py's B200 arm
+    python tools/dryrun_bench.py lora                         # tools/bench_lora.py
 
 The C-ABI is replaced by the torch test double (tests/cabi_double.py), `device="cuda"` is dropped, CUDA events / graphs / clock
 sampling are stubs, and the model is shrunk to toy dimensions.  What this exercises is the DRIVER LOGIC the round-end run depends
@@ -122,7 +122,7 @@ def main():
     bench.ClockSampler = _Clocks
     if which == "decode":
         ChatTSConfig.chatts_14b = _toy(ChatTSConfig.chatts_14b, 2)
-        sys.argv = ["bench.py", "--steps", "2", "--warmup", "1", "--batch", "2", "--no-cpu-baseline"]
+        sys.argv = ["bench.py", "--steps", "2", "--warmup", "1", "--batch", "2", "--no-cpu-baseline"] + sys.argv[2:]      # later flags win
         bench.main()
     else:
         ChatTSConfig.chatts_8b = _toy(ChatTSConfig.chatts_8b, 1)
