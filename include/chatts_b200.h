@@ -172,6 +172,12 @@ int cts_attn_prefill(cts_ctx* ctx, const void* q, const void* k, const void* v, 
  *   seq_lens int32[batch] (tokens incl. the current one); out [batch, nh*d]
  *   workspace: fp32, cts_attn_decode_workspace_floats(...) elements, ZERO-FILLED ONCE by the caller (it holds the
  *   self-resetting arrival counters after the partials)
+ * Preconditions:
+ *   - the kernel this one follows on the stream (its programmatic-dependent-launch predecessor) may write only q and row
+ *     seq_len - 1 of each sequence's K and V: the KV tiles before the one holding that row are loaded ahead of the dependency
+ *     wait, and seq_lens / page_table are read there too, so they must not change inside the step either;
+ *   - every cache row past seq_len that a sequence's last 64-token tile covers (the rest of its last page and the pages the
+ *     table lists after it) must hold finite values: masked keys get probability 0, and 0 times a non-finite value is NaN.
  */
 long long cts_attn_decode_workspace_floats(int batch, int nh, int head_dim, int num_splits);
 int cts_attn_decode(cts_ctx* ctx, const void* q, const void* k_cache, const void* v_cache, int num_pages,

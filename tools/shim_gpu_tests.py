@@ -113,6 +113,9 @@ SELECT = {
     "test_gpu_attention.py": None,                       # calibration: tcgen05 prefill attention (MN-major V operand), HMMA prefill, TMA paged decode (ldmatrix / mma.sync)
     "test_gpu_zz_d_attn_bwd_tc5.py": None,               # tcgen05 attention backward (K-major and MN-major operands, TMEM-resident dQ / dK / dV)
     "test_gpu_w4.py": "not (27648 or 13824 or 7168)",    # both W4A16 kernels (tcgen05 operand path; registers + mma.sync over the persistent schedule), small shapes
+    # aimed queries against the float64 reference: both prefill kernels on the varlen batch, the decode kernel over contexts up to 4097
+    # (no split, the model's split, 32 splits, more splits than tiles) and its PDL predecessor's row
+    "test_gpu_attention_aimed.py": "(varlen and (5-1-d128-tc5-bf16 or 4-1-d64-wmma64-bf16)) or (decode_aimed and 8-2-d64-16 and bf16) or pdl",
 }
 
 # --quick: a subset that finishes in about a minute (what tests/test_shim_kernels.py runs inside the CPU suite)
