@@ -31,6 +31,7 @@ SYMBOLS = [
     "cts_sample_advance", "cts_rmsnorm", "cts_lm_head", "cts_decoder_step_ws_floats", "cts_decoder_step", "cts_ts_encode", "cts_gemm_decode_fused",
     "cts_peer_ll_region_bytes", "cts_peer_allreduce_ll", "cts_trace_enable", "cts_ts_encode_fused_ok", "cts_ts_encode_fused",
     "cts_rep_penalty_mark", "cts_rep_penalty_apply", "cts_gemm_w4", "cts_gemm_w4_suggest_split", "cts_gemm_w4_mma", "cts_gemm_w4_mma_suggest_split",
+    "cts_gemm_w4_prefill",
 ]
 FUSED_RESIDUAL, FUSED_SWIGLU, FUSED_QKV_ROPE = 0, 1, 2
 PACK_DESC_LONGS = 12
@@ -93,6 +94,12 @@ class GemmW4Args(C.Structure):
     _fields_ = [("qw", C.c_void_p), ("scales", C.c_void_p), ("zeros", C.c_void_p), ("x", C.c_void_p), ("out", C.c_void_p),
                 ("n", C.c_longlong), ("k", C.c_longlong), ("t", C.c_longlong), ("x_ld", C.c_longlong),
                 ("group_size", C.c_int), ("split_k", C.c_int), ("dtype", C.c_int), ("reserved", C.c_int)]
+
+
+class GemmW4pArgs(C.Structure):
+    _fields_ = [("qw", C.c_void_p), ("szp", C.c_void_p), ("x", C.c_void_p), ("bias", C.c_void_p), ("residual", C.c_void_p), ("out", C.c_void_p),
+                ("n", C.c_longlong), ("k", C.c_longlong), ("t", C.c_longlong), ("x_ld", C.c_longlong), ("out_ld", C.c_longlong),
+                ("group_size", C.c_int), ("split_k", C.c_int), ("dtype", C.c_int), ("epilogue", C.c_int)]
 
 
 class GemmW4fArgs(C.Structure):
@@ -158,6 +165,7 @@ def load_library():
     lib.cts_gemm_w4_suggest_split.argtypes = [vp, ll, ll]
     lib.cts_gemm_w4_mma.argtypes = [vp, C.POINTER(GemmW4fArgs), vp]
     lib.cts_gemm_w4_mma_suggest_split.argtypes = [vp, ll, ll, ll]
+    lib.cts_gemm_w4_prefill.argtypes = [vp, C.POINTER(GemmW4pArgs), vp]
     lib.cts_rep_penalty_mark.argtypes = [vp, vp, vp, i, vp, i, ll, vp]
     lib.cts_rep_penalty_apply.argtypes = [vp, vp, ll, ll, i, vp, i, f, i, vp]
     lib.cts_ts_encode_fused_ok.argtypes = [C.POINTER(TsEncodeArgs)]
@@ -349,6 +357,20 @@ class Context:
 
     def gemm_w4_mma_suggest_split(self, n, k, t=1):
         return int(self.lib.cts_gemm_w4_mma_suggest_split(self.h, n, k, t))
+
+    def gemm_w4_prefill(self, x, qwf, szp, n, group_size, out, *, bias=None, residual=None, epilogue=EPI_NONE, split_k=1, t=None):
+        """cts_gemm's epilogues (NONE / RESIDUAL / SWIGLU_IL / PARTIAL_F32) over the fragment-major 4-bit weight of gemm_w4_mma
+        (cts_gemm_w4_prefill: persistent tcgen05 GEMM, any t): bit-identical to gemm() on weights.py:dequantize_w4 of the same codes."""
+        a = GemmW4pArgs()
+        a.qw, a.szp, a.x, a.out = qwf.data_ptr(), szp.data_ptr(), x.data_ptr(), out.data_ptr()
+        a.bias = bias.data_ptr() if bias is not None else None
+        a.residual = residual.data_ptr() if residual is not None else None
+        a.n, a.k = int(n), szp.shape[1] * int(group_size)
+        a.t = x.shape[0] if t is None else t
+        a.x_ld = x.stride(0)
+        a.out_ld = out.stride(-2) if epilogue != EPI_PARTIAL_F32 else a.n
+        a.group_size, a.split_k, a.dtype, a.epilogue = int(group_size), int(split_k), dtype_code(x.dtype), int(epilogue)
+        self._chk(self.lib.cts_gemm_w4_prefill(self.h, C.byref(a), _stream()))
 
     # ------------------------------------------------------------------ fused split-K tails
     def reduce_bias_act(self, partial, split_k, t, n, bias, act, out, row_map=None):

@@ -16,7 +16,7 @@ OBJ = os.path.join(CSRC, "_build")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libchatts_b200.so")
 SOURCES = ["ctx.cu", "gemm_tcgen05.cu", "ts_frontend.cu", "elementwise.cu", "attention.cu", "allreduce.cu", "decode_chain.cu",
-           "train_elementwise.cu", "attention_bwd.cu", "sampling.cu", "decoder_step.cu", "attention_bwd_tc5.cu", "lora_wgrad_mma.cu", "gemm_decode_fused.cu", "allreduce_ll.cu", "ts_encoder_fused.cu", "gemm_w4.cu", "gemm_w4_mma.cu"]
+           "train_elementwise.cu", "attention_bwd.cu", "sampling.cu", "decoder_step.cu", "attention_bwd_tc5.cu", "lora_wgrad_mma.cu", "gemm_decode_fused.cu", "allreduce_ll.cu", "ts_encoder_fused.cu", "gemm_w4.cu", "gemm_w4_mma.cu", "gemm_w4_persistent.cu"]
 HEADERS = ["common.cuh", "tensormap.cuh", "trace.cuh", "ts_rows.cuh", os.path.join("..", "..", "include", "chatts_b200.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC",

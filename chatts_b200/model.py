@@ -65,7 +65,9 @@ class _Step:
 class ChatTSForCausalLM:
     def __init__(self, config, state_dict, device="cuda", dtype=torch.bfloat16, tp_rank=0, tp_size=1,
                  max_batch=32, max_seq_len=2048, page_size=64, use_cuda_graph=True, comm=None,
-                 use_peer_allreduce=True, graph_with_tp=True, use_chain=None, use_sample_kernel=None, use_native_step=None, use_fused_decode=None, use_peer_ll=None):
+                 use_peer_allreduce=True, graph_with_tp=True, use_chain=None, use_sample_kernel=None, use_native_step=None, use_fused_decode=None, use_peer_ll=None, dense_projections=True):
+        """dense_projections=False: the decoder projections (q/k/v/o/gate/up/down weights) are not loaded from ``state_dict``; the
+        model is unusable until attach_w4(..., w4_only=True) supplies them as 4-bit weights (from_pretrained(path, w4_only=True))."""
         if not torch.cuda.is_available():
             raise _cabi.CtsError("chatts_b200 needs a B200 (sm_100a) GPU; there is no CPU fallback")
         self.config, self.dtype = config, dtype
@@ -76,6 +78,7 @@ class ChatTSForCausalLM:
         assert cfg.num_key_value_heads % tp_size == 0 and cfg.num_attention_heads % tp_size == 0
         self.nh, self.nkv, self.d = cfg.num_attention_heads // tp_size, cfg.num_key_value_heads // tp_size, cfg.head_dim
         self.H, self.I = cfg.hidden_size, cfg.intermediate_size // tp_size
+        self.n_qkv = (self.nh + 2 * self.nkv) * self.d             # fused q|k|v output features (per rank)
         self.V = cfg.vocab_size // tp_size if tp_size > 1 else cfg.vocab_size
         self.L = cfg.num_hidden_layers
         self.eps = float(cfg.rms_norm_eps)
@@ -117,7 +120,8 @@ class ChatTSForCausalLM:
         # GEMM's stream through L2, so the bytes are read twice.  CTS_NEXT_PREFETCH_MB=<n> turns it on for experiments.
         self.next_prefetch_bytes = int(float(_os.environ.get("CTS_NEXT_PREFETCH_MB", "0")) * (1 << 20))
         self.w4 = None               # W4A16 decode weights (csrc/gemm_w4.cu): set by attach_w4 / quantize_w4_synthetic / from_pretrained(GPTQ)
-        self._load(state_dict)
+        self.w4_only = False         # True: the 4-bit copy is the ONLY copy of the projections (attach_w4(..., w4_only=True))
+        self._load(state_dict, dense_projections)
         # every position the page table can address has a row in the rotary tables (max_pages * page_size >= max_seq_len), capped by
         # the model's max_position_embeddings; _alloc_pages rejects sequences beyond it (no silent out-of-bounds cos/sin read)
         n_pos = min(cfg.max_position_embeddings, max(self.max_pages * page_size, 16))
@@ -134,7 +138,7 @@ class ChatTSForCausalLM:
             self.peer = PeerBuffers(self.ctx, tp_rank, tp_size, self.peer_tokens, self.H, group=comm)
 
     # ------------------------------------------------------------------------------------------ loading
-    def _load(self, sd):
+    def _load(self, sd, dense_projections=True):
         cfg, dev, dt = self.config, self.device, self.dtype
 
         def take(name):
@@ -152,7 +156,6 @@ class ChatTSForCausalLM:
             p = f"model.layers.{l}."
             self.ln1.append(take(p + "input_layernorm.weight"))
             self.ln2.append(take(p + "post_attention_layernorm.weight"))
-            self.wqkv.append(torch.cat([take(p + f"self_attn.{n}_proj.weight") for n in "qkv"], 0).contiguous())
             if (p + "self_attn.q_proj.bias") in sd:
                 self.bqkv.append(torch.cat([take(p + f"self_attn.{n}_proj.bias") for n in "qkv"], 0).contiguous())
             else:
@@ -160,6 +163,11 @@ class ChatTSForCausalLM:
             has_qkn = (p + "self_attn.q_norm.weight") in sd          # Qwen3 / ChatTS-8B
             self.qn.append(take(p + "self_attn.q_norm.weight") if has_qkn else None)
             self.kn.append(take(p + "self_attn.k_norm.weight") if has_qkn else None)
+            if not dense_projections:
+                for lst in (self.wqkv, self.wo, self.wgu, self.wd):
+                    lst.append(None)
+                continue
+            self.wqkv.append(torch.cat([take(p + f"self_attn.{n}_proj.weight") for n in "qkv"], 0).contiguous())
             self.wo.append(take(p + "self_attn.o_proj.weight"))
             # gate/up INTERLEAVED per 128-row tile (64 gate rows, then the 64 matching up rows): SwiGLU becomes local to
             # one MMA tile (CTS_EPI_SWIGLU_IL in the persistent prefill GEMM; cts_reduce_swiglu(interleaved) at decode)
@@ -180,14 +188,18 @@ class ChatTSForCausalLM:
         return cls(config, sd, device=device, dtype=dtype, **kw)
 
     @classmethod
-    def from_pretrained(cls, path, device_map=None, torch_dtype=None, trust_remote_code=True, device=None, **kw):
-        """AutoModelForCausalLM.from_pretrained surface (README.md:88): config.json + safetensors shards."""
+    def from_pretrained(cls, path, device_map=None, torch_dtype=None, trust_remote_code=True, device=None, w4_only=False, **kw):
+        """AutoModelForCausalLM.from_pretrained surface (README.md:88): config.json + safetensors shards.
+        w4_only=True (GPTQ-Int4 checkpoints): the decoder projections are never dequantised; the 4-bit copy is their only copy and serves
+        every step size (attach_w4).  A checkpoint the 4-bit kernels cannot represent raises ValueError instead of loading dense."""
         cfg = ChatTSConfig.from_json(path)
         dt = {"float16": torch.float16, "bfloat16": torch.bfloat16, torch.float16: torch.float16,
               torch.bfloat16: torch.bfloat16, None: getattr(torch, cfg.torch_dtype, torch.bfloat16)}[torch_dtype]
         dev = device if device is not None else (f"cuda:{device_map}" if isinstance(device_map, int) else (device_map or "cuda"))
         sd = load_checkpoint(path, device="cpu")
         w4_packed, w4_gs = None, 0
+        if w4_only and not any(k.endswith(".qweight") for k in sd):
+            raise ValueError("w4_only=True needs a GPTQ-Int4 checkpoint (no *.qweight tensors found)")
         if any(k.endswith(".qweight") for k in sd):                # GPTQ-Int4 checkpoint (README.md:52,262-263)
             import json as _json
             import os as _os
@@ -197,12 +209,20 @@ class ChatTSForCausalLM:
             # decode streams the 4-bit codes (csrc/gemm_w4.cu); prefill runs on a dequantised copy holding the same values (the scales
             # rounded to the model dtype, which is what the kernel multiplies with).  Act-order checkpoints, tensor parallelism and
             # CTS_W4=0 keep the dequantised weights only.
+            if w4_only and (kw.get("tp_size", 1) != 1 or _os.environ.get("CTS_W4", "1") == "0"):
+                raise ValueError("w4_only=True is single-GPU and needs the 4-bit kernels (tp_size=1, CTS_W4 not 0)")
             if _os.environ.get("CTS_W4", "1") != "0" and kw.get("tp_size", 1) == 1:
                 w4_packed, w4_gs = gptq_w4_pack(sd, qc, dtype=dt)
+            if w4_only:
+                if w4_packed is None:
+                    raise ValueError("w4_only=True: this GPTQ checkpoint cannot be represented by the 4-bit kernels (act-order g_idx, "
+                                     "a group size that is not a multiple of 64 or differs between projections, or not 4-bit)")
+                # the packed decoder projections never become dense; other quantised tensors (if any) are dequantised as before
+                sd = {k: t for k, t in sd.items() if not (k.rsplit(".", 1)[0] in w4_packed and k.rsplit(".", 1)[1] in ("qweight", "qzeros", "scales", "g_idx"))}
             sd = dequantize_gptq(sd, qc, dtype=dt, scale_dtype=dt if w4_packed is not None else None)
-        model = cls(cfg, sd, device=dev, dtype=dt, **kw)
+        model = cls(cfg, sd, device=dev, dtype=dt, dense_projections=not w4_only, **kw)
         if w4_packed is not None:
-            model.attach_w4(w4_packed, w4_gs)
+            model.attach_w4(w4_packed, w4_gs, w4_only=w4_only)
         # generation_config.json: the defaults HF's generate() applies when the caller passes none (README.md:102 calls
         # model.generate(**inputs, max_new_tokens=300) with no sampling arguments)
         import json as _json2
@@ -224,6 +244,8 @@ class ChatTSForCausalLM:
         import json
         import os
         import re
+        if self.w4_only:
+            raise ValueError("merge_lora needs the dense projection weights: this model keeps its projections as 4-bit weights only (w4_only)")
         if isinstance(adapter, str):
             cfg_path = os.path.join(adapter, "adapter_config.json")
             if os.path.exists(cfg_path):
@@ -276,15 +298,21 @@ class ChatTSForCausalLM:
         return merged          # in-place update: captured decode graphs keep reading the same (now merged) buffers
 
     # ------------------------------------------------------------------------------------------ W4A16 (GPTQ-Int4, README.md:52,262-263)
-    def attach_w4(self, packed, group_size):
+    def attach_w4(self, packed, group_size, w4_only=False):
         """Switch the DECODE step to the 4-bit weight stream.  ``packed``: {HF linear name (e.g. 'model.layers.3.mlp.up_proj'):
         (qw uint8 [out, in/2], scales [out, in/g], zeros uint8 [out, in/g])} in the layout of weights.py:repack_gptq_w4, for all
         seven projections of every layer.  The dense weights stay (prefill and every T > 32 step use them): they must hold the SAME
         values, i.e. weights.py:dequantize_gptq(..., scale_dtype=model dtype) -- 180 GB of HBM keep both copies.  Fused operands
         are assembled exactly like the dense ones: q|k|v stacked, gate/up interleaved per 64 rows.  Single GPU (a tensor-parallel
-        row split would cut groups: down_proj's 13824 / 8 = 1728 inputs are not a multiple of the group size)."""
+        row split would cut groups: down_proj's 13824 / 8 = 1728 inputs are not a multiple of the group size).
+        w4_only=True: the 4-bit copy becomes the ONLY copy of the projections -- the dense wqkv / wo / wgu / wd are freed and every step
+        size runs from the fragment-major codes (T <= 32 decode: cts_gemm_w4_mma; everything else: cts_gemm_w4_prefill with the epilogue
+        and split factor the dense path uses, bit-identical to it).  Refused for shapes the fragment-major kernels cannot take, with the
+        fused decode (use_fused_decode), and later by merge_lora and train.LoraTrainer, which need dense weights."""
         if self.tp_size != 1:
             raise ValueError("W4A16 decode weights are single-GPU (tensor parallelism uses the dequantised weights)")
+        if w4_only and self.use_fused_decode:
+            raise ValueError("w4_only=True: the fused decode GEMMs (use_fused_decode) read dense weights; build the model with use_fused_decode=0")
         dev = self.device
         gs = int(group_size)
         w4 = dict(group_size=gs, qkv=[], o=[], gu=[], d=[])
@@ -311,7 +339,11 @@ class ChatTSForCausalLM:
         # dense GEMM, no faster than it: kept as the checker)
         w4["kernel"] = _os.environ.get("CTS_W4_KERNEL", "mma")
         k_dims = (self.H, self.nh * self.d, self.I)
-        if w4["kernel"] == "mma" and not (all(kd % 128 == 0 for kd in k_dims) and (gs == 64 or gs % 128 == 0)):
+        mma_ok = all(kd % 128 == 0 for kd in k_dims) and (gs == 64 or gs % 128 == 0)
+        if w4_only and not (mma_ok and w4["kernel"] == "mma"):
+            raise ValueError(f"w4_only=True needs the fragment-major 4-bit layout: every K ({k_dims}) a multiple of 128, group size 64 or a "
+                             f"multiple of 128 (got {gs}), and CTS_W4_KERNEL=mma")
+        if w4["kernel"] == "mma" and not mma_ok:
             w4["kernel"] = "tc5"          # the mma kernel's pipeline stage is 128 K wide (cts_gemm_w4f_args): odd shapes take the tcgen05 kernel
         if w4["kernel"] == "mma":
             from .weights import repack_w4_mma
@@ -321,16 +353,24 @@ class ChatTSForCausalLM:
                     w4[kind][l] = repack_w4_mma(qw, sc, zp, gs) + (int(qw.shape[0]),)
             w4["splits"] = None           # per batch size: _w4_splits
         else:
-            w4["splits"] = dict(qkv=c.gemm_w4_suggest_split(self.wqkv[0].shape[0], self.H), o=c.gemm_w4_suggest_split(self.H, self.nh * self.d),
+            w4["splits"] = dict(qkv=c.gemm_w4_suggest_split(self.n_qkv, self.H), o=c.gemm_w4_suggest_split(self.H, self.nh * self.d),
                                 gu=c.gemm_w4_suggest_split(2 * self.I, self.H), d=c.gemm_w4_suggest_split(self.H, self.I))
+        w4["only"] = bool(w4_only)
         self.w4 = w4
+        if w4_only:
+            # no dense copy: nothing may reach for one (None fails loudly), and no GEMM names a dense weight as its L2-prefetch successor
+            for lst in (self.wqkv, self.wo, self.wgu, self.wd):
+                lst[:] = [None] * self.L
+            self.w4_only = True
+            self.next_prefetch_bytes = 0
+            self.__dict__.pop("_layer_list", None)          # the native step's cached operand list would keep the dense weights alive
         self._steps = {}                  # decode states (workspaces, captured graphs) are rebuilt for the new launches
         return self
 
-    def quantize_w4_synthetic(self, group_size=128, seed=7):
+    def quantize_w4_synthetic(self, group_size=128, seed=7, w4_only=False):
         """Benchmark / test helper (no GPTQ checkpoint exists offline): draw random 4-bit codes, scales and zero points at the model's
         shapes, REPLACE the dense weights by their dequantised values and attach the packed copy -- a W4A16 model whose prefill and
-        decode paths see the same weights."""
+        decode paths see the same weights.  w4_only=True: the same codes (same seed), attached as the only copy (attach_w4)."""
         from .weights import dequantize_w4, W4_NIBBLE_OF_K  # noqa: F401
         g = torch.Generator(device=self.device).manual_seed(seed)
         packed = {}
@@ -349,14 +389,17 @@ class ChatTSForCausalLM:
                                         ("self_attn.o_proj", (H, self.nh * d)), ("mlp.gate_proj", (I, H)), ("mlp.up_proj", (I, H)), ("mlp.down_proj", (H, I))):
                 t = make(n_out, n_in)
                 packed[p + name] = t
-                parts[name] = dequantize_w4(*t, group_size)
+                if not w4_only:
+                    parts[name] = dequantize_w4(*t, group_size)
+            if w4_only:
+                continue
             self.wqkv[l].copy_(torch.cat([parts["self_attn.q_proj"], parts["self_attn.k_proj"], parts["self_attn.v_proj"]], 0))
             self.wo[l].copy_(parts["self_attn.o_proj"])
             gp, up = parts["mlp.gate_proj"], parts["mlp.up_proj"]
             self.wgu[l].copy_(torch.stack([gp.view(-1, 64, H), up.view(-1, 64, H)], 1).reshape(2 * I, H))
             self.wd[l].copy_(parts["mlp.down_proj"])
             del parts
-        return self.attach_w4(packed, group_size)
+        return self.attach_w4(packed, group_size, w4_only=w4_only)
 
     # ------------------------------------------------------------------------------------------ layers
     def _splits(self, T):
@@ -366,11 +409,11 @@ class ChatTSForCausalLM:
         if ov and T <= 32:
             a = [int(v) for v in ov.split(",")]
             return dict(qkv=a[0], o=a[1], gu=a[2], d=a[3])
-        return dict(qkv=c.suggest_split(self.wqkv[0].shape[0], self.H, T), o=c.suggest_split(self.H, self.nh * self.d, T),
+        return dict(qkv=c.suggest_split(self.n_qkv, self.H, T), o=c.suggest_split(self.H, self.nh * self.d, T),
                     gu=c.suggest_split(self.I, self.H, T, True), d=c.suggest_split(self.H, self.I, T))
 
     def _ws_floats(self, T, sp):
-        return max(sp["qkv"] * T * self.wqkv[0].shape[0] if sp["qkv"] > 1 else 0, sp["o"] * T * self.H if sp["o"] > 1 else 0,
+        return max(sp["qkv"] * T * self.n_qkv if sp["qkv"] > 1 else 0, sp["o"] * T * self.H if sp["o"] > 1 else 0,
                    sp["gu"] * T * 2 * self.I if T <= 128 else 0, sp["d"] * T * self.H if sp["d"] > 1 else 0, 1)
 
     def _w4_splits(self, T):
@@ -378,7 +421,7 @@ class ChatTSForCausalLM:
         w4, c = self.w4, self.ctx
         if w4["splits"] is not None:
             return w4["splits"]
-        return dict(qkv=c.gemm_w4_mma_suggest_split(self.wqkv[0].shape[0], self.H, T), o=c.gemm_w4_mma_suggest_split(self.H, self.nh * self.d, T),
+        return dict(qkv=c.gemm_w4_mma_suggest_split(self.n_qkv, self.H, T), o=c.gemm_w4_mma_suggest_split(self.H, self.nh * self.d, T),
                     gu=c.gemm_w4_mma_suggest_split(2 * self.I, self.H, T), d=c.gemm_w4_mma_suggest_split(self.H, self.I, T))
 
     def _layers(self, st, T, attend):
@@ -394,6 +437,18 @@ class ChatTSForCausalLM:
         w4 = self.w4 if (self.w4 is not None and T <= 32 and st.k_lin is None and not fused) else None
         if w4 is not None:
             sp = self._w4_splits(T)
+        # 4-bit-only models: every other step (prefill of any length, decode batches of 33-128 rows) runs the projections through
+        # cts_gemm_w4_prefill with exactly the epilogue and split factor the dense path below chooses -- the same numbers, bit for bit
+        w4p = self.w4 if (self.w4 is not None and self.w4["only"] and w4 is None) else None
+
+        def gemm(kind, l, x, w, out, **kw):
+            """One projection: the dense GEMM on ``w``, or the 4-bit weight of (kind, l) with the same epilogue (4-bit-only models)."""
+            if w4p is None:
+                c.gemm(x, w, out, **kw)
+                return
+            qwf, szp, n_out = w4p[kind][l]
+            kw = {k: v for k, v in kw.items() if not k.startswith("next_")}
+            c.gemm_w4_prefill(x, qwf, szp, n_out, w4p["group_size"], out, **kw)
 
         def proj(kind, l, x, w, split, **kw):
             """fp32 split-K partials of one projection into st.ws: from the packed 4-bit weight when attached, else from the dense one."""
@@ -404,7 +459,7 @@ class ChatTSForCausalLM:
                 qw, sc, zp = w4[kind][l]
                 c.gemm_w4(x, qw, sc, zp, w4["group_size"], st.ws, split, t=T)
             else:
-                c.gemm(x, w, st.ws, epilogue=EPI_PARTIAL_F32, split_k=split, t=T, **kw)
+                gemm(kind, l, x, w, st.ws, epilogue=EPI_PARTIAL_F32, split_k=split, t=T, **kw)
 
         def nxt(w, split):
             return dict(next_w=w, next_split=split, next_bytes=nb) if nb > 0 else {}
@@ -466,7 +521,7 @@ class ChatTSForCausalLM:
                 c.qkv_rope_cache(st.ws, True, sp["qkv"], self.bqkv[l], st.positions, self.cos, self.sin, st.slot_map, st.q, kc, vc,
                                  st.k_lin, st.v_lin, T, self.nh, self.nkv, self.d, self.page_size, self.qn[l], self.kn[l], eps)
             else:
-                c.gemm(st.xn, self.wqkv[l], st.qkv, bias=self.bqkv[l], epilogue=EPI_NONE, t=T, **nxt(self.wo[l], sp["o"]))
+                gemm("qkv", l, st.xn, self.wqkv[l], st.qkv, bias=self.bqkv[l], epilogue=EPI_NONE, t=T, **nxt(self.wo[l], sp["o"]))
                 c.qkv_rope_cache(st.qkv, False, 1, None, st.positions, self.cos, self.sin, st.slot_map, st.q, kc, vc,
                                  st.k_lin, st.v_lin, T, self.nh, self.nkv, self.d, self.page_size, self.qn[l], self.kn[l], eps)
             attend(l)
@@ -477,11 +532,11 @@ class ChatTSForCausalLM:
                 proj("o", l, st.ao, self.wo[l], sp["o"], **nxt(self.wgu[l], sp["gu"]))
                 c.reduce_residual_rmsnorm(st.ws, sp["o"], st.h, st.h, self.ln2[l], eps, st.xn, t=T)
             else:
-                c.gemm(st.ao, self.wo[l], st.h, residual=st.h, epilogue=EPI_RESIDUAL, t=T, **nxt(self.wgu[l], sp["gu"]))
+                gemm("o", l, st.ao, self.wo[l], st.h, residual=st.h, epilogue=EPI_RESIDUAL, t=T, **nxt(self.wgu[l], sp["gu"]))
                 c.reduce_residual_rmsnorm(None, 0, st.h, None, self.ln2[l], eps, st.xn, t=T)
             # ---- gate/up + SwiGLU
             if T > 128:
-                c.gemm(st.xn, self.wgu[l], st.act, epilogue=EPI_SWIGLU_IL, t=T)          # persistent, SwiGLU fused in the tile
+                gemm("gu", l, st.xn, self.wgu[l], st.act, epilogue=EPI_SWIGLU_IL, t=T)   # persistent, SwiGLU fused in the tile
             else:
                 proj("gu", l, st.xn, self.wgu[l], sp["gu"], **nxt(self.wd[l], sp["d"]))
                 c.reduce_swiglu(st.ws, sp["gu"], T, I, st.act, interleaved=True)
@@ -494,7 +549,7 @@ class ChatTSForCausalLM:
                 proj("d", l, st.act, self.wd[l], sp["d"], **after)
                 c.reduce_residual_rmsnorm(st.ws, sp["d"], st.h, st.h, nw, eps, st.xn, t=T)
             else:
-                c.gemm(st.act, self.wd[l], st.h, residual=st.h, epilogue=EPI_RESIDUAL, t=T, **after)
+                gemm("d", l, st.act, self.wd[l], st.h, residual=st.h, epilogue=EPI_RESIDUAL, t=T, **after)
                 c.reduce_residual_rmsnorm(None, 0, st.h, None, nw, eps, st.xn, t=T)
 
     def _tp_row_parallel(self, st, T, x, w, norm_w, which, split, nxt=None):
@@ -561,14 +616,14 @@ class ChatTSForCausalLM:
             st.tp_proj = torch.empty(tp_pad, self.H, device=dev, dtype=dt)
             st.tp_shard32 = torch.empty(ct * self.H, device=dev, dtype=torch.float32)
             st.tp_shard16 = torch.empty(ct * self.H, device=dev, dtype=dt)
-        st.qkv = torch.empty(T, self.wqkv[0].shape[0], device=dev, dtype=dt) if st.splits["qkv"] == 1 else None
+        st.qkv = torch.empty(T, self.n_qkv, device=dev, dtype=dt) if st.splits["qkv"] == 1 else None
         ws_n = max(self._ws_floats(T, st.splits), T * self.H, tp_pad * self.H)
         if decode and self.w4 is not None and T <= 32:   # W4A16 decode: every projection through the partial path with the W4 split factors
             sp = self._w4_splits(T)
-            ws_n = max(ws_n, sp["qkv"] * T * self.wqkv[0].shape[0], sp["o"] * T * self.H, sp["gu"] * T * 2 * self.I, sp["d"] * T * self.H)
+            ws_n = max(ws_n, sp["qkv"] * T * self.n_qkv, sp["o"] * T * self.H, sp["gu"] * T * 2 * self.I, sp["d"] * T * self.H)
         if decode and self.use_native_step:          # cts_decoder_step always takes the split-K partial path (also at factor 1)
             sp = st.splits
-            ws_n = max(ws_n, sp["qkv"] * T * self.wqkv[0].shape[0], sp["o"] * T * self.H, sp["gu"] * T * 2 * self.I, sp["d"] * T * self.H)
+            ws_n = max(ws_n, sp["qkv"] * T * self.n_qkv, sp["o"] * T * self.H, sp["gu"] * T * 2 * self.I, sp["d"] * T * self.H)
         st.ws = torch.empty(ws_n, device=dev, dtype=torch.float32)                           # split-K partials [S, T, N]
         st.positions = torch.zeros(T, device=dev, dtype=torch.int32)
         st.slot_map = torch.zeros(T, device=dev, dtype=torch.int32)

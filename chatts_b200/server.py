@@ -362,6 +362,8 @@ def main():
     ap.add_argument("--scheduler", default="batch", choices=["batch", "continuous"],
                     help="batch: micro-batches run to completion (sampling supported); continuous: iteration-level batching, greedy")
     ap.add_argument("--steps-per-round", type=int, default=4, help="continuous scheduler: decode steps between two host reads")
+    ap.add_argument("--w4-only", action="store_true",
+                    help="GPTQ-Int4 checkpoint: keep the decoder projections as 4-bit weights only (no dense copy; frees HBM for KV cache)")
     args = ap.parse_args()
     import uvicorn
     from .vllm_compat import LLM
@@ -371,7 +373,7 @@ def main():
         from transformers import AutoTokenizer
         tok = AutoTokenizer.from_pretrained(args.model, trust_remote_code=True)
     llm = LLM(model=args.model, tokenizer=tok, dtype=args.dtype, max_model_len=args.max_model_len, max_num_seqs=args.max_num_seqs,
-              limit_mm_per_prompt={"timeseries": limit})
+              limit_mm_per_prompt={"timeseries": limit}, w4_only=args.w4_only)
     uvicorn.run(create_app(llm, args.served_model_name, args.batch_window_ms, limit, args.scheduler, args.steps_per_round),
                 host=args.host, port=args.port)
 

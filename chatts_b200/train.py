@@ -75,6 +75,8 @@ class LoraTrainer:
                  weight_decay=0.0, max_grad_norm=1.0, seed=0, init_b_std=0.0, group=None, adapters=None):
         if model.tp_size != 1:
             raise ValueError("LoraTrainer is data parallel: build the model with tp_size=1 on every rank")
+        if getattr(model, "w4_only", False):
+            raise ValueError("LoraTrainer needs the dense projection weights: this model keeps its projections as 4-bit weights only (w4_only)")
         if not 1 <= int(r) <= 64:
             raise ValueError("LoRA rank must be in [1, 64]")
         self.model, self.ctx = model, model.ctx

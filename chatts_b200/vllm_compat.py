@@ -141,13 +141,14 @@ def _make_llm(**kw):
 class LLM:
     def __init__(self, model=None, tokenizer=None, config=None, state_dict=None, tensor_parallel_size=1, dtype="bfloat16",
                  max_model_len=2048, max_num_seqs=32, limit_mm_per_prompt=None, trust_remote_code=True, seed=1234,
-                 distributed_backend="nccl", **kw):
+                 distributed_backend="nccl", w4_only=False, **kw):
         """tensor_parallel_size = k > 1 (every caller of the reference passes it: demo/demo_vllm.py:30, llm_utils.py:153-154):
           * under torchrun / an initialised process group of k ranks the engine ATTACHES: every rank constructs the LLM and makes the
             same generate() calls (rank r holds shard r);
           * otherwise the constructor SPAWNS k - 1 worker processes (one per GPU, as vLLM's multiprocessing executor does,
             README.md:141) that build their shards and mirror every generate() call of this process (rank 0) -- the model must then
-            be named by a path or by config + seed (a ChatTSForCausalLM instance cannot be sent to another process)."""
+            be named by a path or by config + seed (a ChatTSForCausalLM instance cannot be sent to another process).
+        w4_only=True: a GPTQ-Int4 checkpoint path is loaded with its projections as 4-bit weights only (from_pretrained(w4_only=True))."""
         import os
         self._tp_procs, self._tp_driver = [], False
         tp = int(tensor_parallel_size or 1)
@@ -193,7 +194,8 @@ class LLM:
         if isinstance(model, ChatTSForCausalLM):
             self.model = model
         elif isinstance(model, str):
-            self.model = ChatTSForCausalLM.from_pretrained(model, torch_dtype=dt, max_seq_len=max_model_len, max_batch=max_num_seqs, **tp_kw)
+            self.model = ChatTSForCausalLM.from_pretrained(model, torch_dtype=dt, max_seq_len=max_model_len, max_batch=max_num_seqs,
+                                                           w4_only=w4_only, **tp_kw)
         else:
             cfg = config or ChatTSConfig.chatts_14b()
             self.model = (ChatTSForCausalLM(cfg, state_dict, dtype=dt, max_seq_len=max_model_len, max_batch=max_num_seqs, **tp_kw)

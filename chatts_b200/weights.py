@@ -233,13 +233,14 @@ def dequantize_gptq(sd, quant_cfg=None, dtype=torch.bfloat16, scale_dtype=None):
 
 def gptq_w4_pack(sd, quant_cfg=None, dtype=torch.bfloat16):
     """({linear name: (qw, scales, zeros)} in the W4A16 kernel's layout, group size) for a GPTQ checkpoint's decoder projections, or
-    (None, 0) when the checkpoint cannot use the kernel: not 4-bit, an act-order g_idx, or a group size that is not a multiple of 64."""
+    (None, 0) when the checkpoint cannot use the kernel: not 4-bit, an act-order g_idx, a group size that is not a multiple of 64, or
+    linears that do not share one group size (group_size -1 = one group per input column: q/k/v/gate/up and o/down differ in n_in)."""
     quant_cfg = quant_cfg or {}
     if int(quant_cfg.get("bits", 4)) != 4:
         return None, 0
     gs = int(quant_cfg.get("group_size", 128))
     zo = 0 if str(quant_cfg.get("checkpoint_format", "gptq")) == "gptq_v2" else 1
-    out = {}
+    out, groups = {}, set()
     for k, t in sd.items():
         if not k.endswith(".qweight") or ".layers." not in k:
             continue
@@ -252,8 +253,8 @@ def gptq_w4_pack(sd, quant_cfg=None, dtype=torch.bfloat16):
         if gi is not None and not torch.equal(gi.to(torch.int64).cpu(), torch.arange(n_in) // group):
             return None, 0                                                # act-order: rows of one group are scattered over K
         out[base] = repack_gptq_w4(t, sd[base + ".qzeros"], sd[base + ".scales"], group, zo, dtype)
-        gs_used = group
-    return (out, gs_used) if out else (None, 0)
+        groups.add(group)
+    return (out, groups.pop()) if out and len(groups) == 1 else (None, 0)
 
 
 def pack_gptq_linear(w, group_size=128, zero_offset=1):

@@ -534,6 +534,25 @@ typedef struct {
 int cts_gemm_w4_mma(cts_ctx* ctx, const cts_gemm_w4f_args* args, void* stream);
 int cts_gemm_w4_mma_suggest_split(cts_ctx* ctx, long long n, long long k, long long t);
 
+/* The W4A16 projection for prefill-sized steps (any t; the model uses it for t > 32) of GPTQ-Int4 checkpoints (README.md:52,262-263):
+ * a persistent tcgen05 GEMM (csrc/gemm_w4_persistent.cu) that dequantises the SAME fragment-major copy cts_gemm_w4_mma streams (qw, szp
+ * exactly as in cts_gemm_w4f_args) into the shared-memory A operand, so a model needs no dense copy of its projections.  Epilogues with
+ * cts_gemm's semantics, and results BIT-IDENTICAL to cts_gemm on the dequantised weight (weights.py:dequantize_w4):
+ *   CTS_EPI_NONE         out[t][n] = dtype(acc + bias)                                 (bias optional, [n] model dtype)
+ *   CTS_EPI_RESIDUAL     out[t][n] = dtype(dtype(acc + bias) + residual[t][n])         (residual may alias out; row stride out_ld)
+ *   CTS_EPI_SWIGLU_IL    out[t][j] = dtype(dtype(silu(dtype(gate))) * dtype(up)) over a gate/up weight interleaved per 64 rows
+ *                        (n % 128 == 0, t > 128; out [t, n / 2])
+ *   CTS_EPI_PARTIAL_F32  out = fp32 [split_k, t, n]; split s sums the 64-wide K blocks [kb * s / split_k, kb * (s + 1) / split_k),
+ *                        kb = k / 64 -- cts_gemm's partition, so the cts_reduce_* / cts_qkv_rope_cache tails take either
+ * k % 128 == 0; group_size 64 or a multiple of 128 dividing k; 1 <= split_k <= k / 64 (> 1 only with CTS_EPI_PARTIAL_F32); x rows
+ * 16-byte aligned (x_ld >= k, x_ld % 8 == 0); qw / szp 16-byte aligned.  A failed check returns CTS_ERR_BAD_ARG and launches nothing. */
+typedef struct {
+  const void* qw; const void* szp; const void* x; const void* bias; const void* residual; void* out;
+  long long n, k, t, x_ld, out_ld;
+  int group_size, split_k, dtype, epilogue;
+} cts_gemm_w4p_args;
+int cts_gemm_w4_prefill(cts_ctx* ctx, const cts_gemm_w4p_args* args, void* stream);
+
 /* Repetition penalty (transformers RepetitionPenaltyLogitsProcessor; generation_config.json of a checkpoint may set it): the set of
  * token ids that occur in a row's sequence is a bit mask seen[batch][words_per_row] (words_per_row >= ceil(vocab / 32), zeroed by the
  * caller).  _mark sets the bits of n (row, token) pairs (rows NULL: pair i belongs to row i -- the new token of every sequence after

@@ -59,10 +59,10 @@ torch.cuda.is_available = lambda: True
 torch.cuda.current_device = lambda: 0
 torch.cuda.is_current_stream_capturing = lambda: False
 
-from tests.cuda_on_cpu.shim import shim_context  # noqa: E402
+from tests.w4_prefill_support import shim_context_w4p  # noqa: E402
 import tests.gpu_util as gu  # noqa: E402
 
-_ctx = shim_context()
+_ctx = shim_context_w4p()                  # the standard shim library + csrc/gemm_w4_persistent.cu
 from tests.cabi_double import TorchDouble as _TD  # noqa: E402
 _dbl = _TD()
 # HYBRID context for the whole-step tests: every entry point whose source is in the shim build runs that source; the others (tcgen05
@@ -116,6 +116,8 @@ SELECT = {
     # aimed queries against the float64 reference: both prefill kernels on the varlen batch, the decode kernel over contexts up to 4097
     # (no split, the model's split, 32 splits, more splits than tiles) and its PDL predecessor's row
     "test_gpu_attention_aimed.py": "(varlen and (5-1-d128-tc5-bf16 or 4-1-d64-wmma64-bf16)) or (decode_aimed and 8-2-d64-16 and bf16) or pdl",
+    # the W4A16 prefill GEMM against the dense GEMM, bit for bit, at the small shapes (every epilogue, split-K, both dtypes), and its checks
+    "test_gpu_w4_prefill.py": "small or bad_arguments",
 }
 
 # --quick: a subset that finishes in about a minute (what tests/test_shim_kernels.py runs inside the CPU suite)
